@@ -29,6 +29,11 @@ After the timed region `parity_sample` re-runs a few replicas of the SAME run (s
 CPU oracle and compares their summaries, entity statistics and -- in record mode -- the raw recorder rings
 byte for byte: the number printed is for a run whose results are the reference's.
 
+--steps K times exactly K windows; when --warmup + --steps windows do not fit the horizon, the run continues past it
+(the JSON line reports the horizon used).  --dump-outputs DIR writes what the last timed step left for a caller of
+Engine.read_outputs (see dump_outputs) as float64 .npy files, at most 64 MB in all; the inputs depend only on the
+arguments (--seed), so two builds run with the same arguments can be compared output for output.
+
 --impl reference times the reference's own CPU path on the host cores: the UNMODIFIED Python reference
 (installed by the recipe in DESIGN.md section 8 into baseline/_ref, which travels to the GPU box) through its
 own ParallelRunner(max_workers=cores).run_replicas, kind "reference"; if that install is missing, the C
@@ -48,6 +53,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
+sys.dont_write_bytecode = True          # the bench runs from a built tree and leaves it as it found it
 
 METRIC = "simulated_events_per_second"
 UNIT = "events/s"
@@ -73,7 +79,12 @@ def parse():
     ap.add_argument("--no-other-mode", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-e2e-records", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float64) for comparing builds")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return a
 
 
 def peaks():
@@ -251,7 +262,6 @@ def cpu_reference_throughput(budget_s, cores, seed):
 def run_reference_arm(a, rank, world):
     if rank != 0:
         return
-    subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle")], stdout=subprocess.DEVNULL)
     cores, core_info = host_cores()
     n_runs = a.steps + a.warmup
     budget = max(2.0, min(8.0, 90.0 / max(1, n_runs)))
@@ -290,6 +300,39 @@ def run_reference_arm(a, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 64 << 20
+DUMP_KEYS = ("summaries", "entity_stats", "records", "sink_samples", "service_samples", "histograms", "sketches")
+
+
+def dump_outputs(out_dir, outs, prefix, budget):
+    """The per-replica outputs a caller of Engine.read_outputs receives, as float64 .npy files: one file per field of a
+    structured array (<key>.<field>.npy; 64-bit unsigned fields, e.g. the order hash, split exactly into .hi / .lo
+    32-bit halves).  Every key gets an equal share of `budget` bytes; a key whose replicas do not all fit keeps a
+    fixed, seeded sample of them, and <key>.replica.npy names the replicas kept, in order."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    keys = [k for k in DUMP_KEYS if outs.get(k) is not None]
+    order = np.random.default_rng(20240601).permutation(len(outs["summaries"]))
+    for k in keys:
+        arr = outs[k]
+        cols = {}
+        for f in (arr.dtype.names or [None]):
+            if f == "pad":
+                continue
+            v = arr if f is None else arr[f]
+            name = k if f is None else f"{k}.{f}"
+            if v.dtype == np.uint64:
+                cols[name + ".hi"], cols[name + ".lo"] = v >> np.uint64(32), v & np.uint64(0xFFFFFFFF)
+            else:
+                cols[name] = v
+        per_replica = 8 * (1 + sum(int(np.prod(c.shape[1:])) for c in cols.values()))
+        keep = min(len(arr), budget // len(keys) // max(1, per_replica))
+        rows = np.arange(len(arr)) if keep == len(arr) else np.sort(order[:keep])
+        np.save(os.path.join(out_dir, f"{prefix}{k}.replica.npy"), rows.astype(np.float64))
+        for name, c in cols.items():
+            np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), np.ascontiguousarray(c[rows], dtype=np.float64))
+
+
 # --------------------------------------------------------------------------- GPU arm
 
 def main():
@@ -320,18 +363,13 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    # the CPU oracle (checker of the parity sample, CPU legs) is built once per node, before any rank loads it
-    if local == 0:
-        subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle")], stdout=subprocess.DEVNULL)
-    barrier()
     cfg = make_config(a)
     model, n = cfg["model"], cfg["replicas"]
     end_ns = int(cfg["horizon_s"] * 1e9)
     win_ns = int(cfg["window_s"] * 1e9)
-    n_windows_max = int(math.ceil(end_ns / win_ns))
-    if a.warmup + a.steps > n_windows_max:
-        raise SystemExit(f"--warmup + --steps = {a.warmup + a.steps} windows exceed the horizon ({n_windows_max} windows "
-                         f"of {cfg['window_s']:g} s); lower --window-s")
+    if (a.warmup + a.steps) * win_ns > end_ns:      # every step asked for is timed: the run continues past the horizon
+        end_ns = (a.warmup + a.steps) * win_ns
+        cfg["horizon_s"] = end_ns / 1e9
     stream = torch.cuda.Stream()
     eng = engine.Engine(local, stream=stream.cuda_stream)
     eng.upload(model)
@@ -382,6 +420,8 @@ def main():
         clk.start()
     res = timed_run(cfg["mode"], a.steps, a.warmup)
     clocks = clk.stop() if rank == 0 else None
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, eng.read_outputs(), f"rank{rank}." if world > 1 else "", DUMP_BYTES // world)
 
     def reduce_max(x):
         if world == 1:

@@ -1,8 +1,8 @@
 """happysim_b200.install(): the reference's own Simulation.run / ParallelRunner.run_replicas routed through the engine.
 
-CPU part (needs the reference importable: /root/reference in the build container or baseline/_ref): models that
-do not lower fall through to the reference's Python loop unchanged; the example's user-defined step profile
-(examples/queuing/m_m_1_queue.py:104-169) tabulates exactly; eligibility rules.
+CPU part: the example's user-defined step profile (examples/queuing/m_m_1_queue.py:104-169) tabulates exactly
+(replayed from its recorded answers, tests/golden/ref_example_step_profile.npz); with the reference importable
+(REF_DIRS): models that do not lower fall through to the reference's Python loop unchanged; eligibility rules.
 GPU part (tests/test_gpu_install.py): the stock-seeded README quick-start gives the reference's own numbers."""
 import importlib.util
 import os
@@ -37,11 +37,25 @@ def _example_module():
     return mod
 
 
+class _RecordedProfile:
+    """The example's MetastableLoadProfile, answering from what the reference answered at the same times: runs of
+    equal rate, first_s[i] <= t <= last_s[i] -> rate[i] (written by tests/golden/gen_example_profile_golden.py)."""
+
+    def __init__(self):
+        z = np.load(os.path.join(ROOT, "tests", "golden", "ref_example_step_profile.npz"))
+        self.first, self.last, self.rate = z["first_s"], z["last_s"], z["rate"]
+
+    def get_rate(self, time):
+        t = time.to_seconds()
+        i = int(np.searchsorted(self.first, t, side="right")) - 1
+        assert i >= 0 and t <= self.last[i], f"the reference was not asked for the rate at t = {t!r}"
+        return float(self.rate[i])
+
+
 def test_example_step_profile_tabulates_exactly():
-    _reference()
     import happysim_b200 as hs
-    from happysimulator import Instant
-    prof = _example_module().MetastableLoadProfile()
+    from happysim_b200 import Instant
+    prof = _RecordedProfile()
     sp = hs.StepProfile.from_profile(prof, end_s=400.0)
     assert list(sp.breakpoints) == [25.0, 30.0, 35.0, 55.0, 60.0, 65.0, 76.0, 87.0, 98.0, 109.0]
     assert list(sp.rates) == [5.0, 15.0, 5.0, 9.0, 15.0, 9.0, 7.0, 6.0, 5.0, 4.0, 3.0]
@@ -53,17 +67,15 @@ def test_example_step_profile_tabulates_exactly():
 
 
 def test_non_step_profile_is_rejected_not_approximated():
-    _reference()
     import happysim_b200 as hs
-    from happysimulator import Profile
 
-    class Ramp(Profile):
+    class Ramp:
         def get_rate(self, time):
             return 5.0 + time.to_seconds()
     with pytest.raises(hs.UnsupportedModelError):
         hs.StepProfile.from_profile(Ramp(), end_s=20.0)
 
-    class TwoChangesInOneScanStep(Profile):
+    class TwoChangesInOneScanStep:
         def get_rate(self, time):
             t = time.to_seconds()
             return 9.0 if 1.0002 <= t < 1.0004 else 5.0
